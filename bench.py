@@ -7,6 +7,7 @@ exactly 128 steps run).  bf16 weights/activations, random-init weights of the re
 
   python bench.py --gpus N --steps K --warmup W          # this repo's CUDA engine (tensor parallel for N > 1)
   python bench.py --impl reference ...                   # the reference's CPU path, bounded sample (rank 0 only)
+  python bench.py ... --dump-outputs DIR                 # also write the last timed step's outputs as DIR/<name>.npy
 
 Prints ONE JSON line (see the task contract): value = device-resident tok/s, e2e = through the public API with host
 buffers, roofline = achieved HBM GB/s of the decode step's weight-streaming kernels vs MEASURED_PEAKS.json,
@@ -102,6 +103,22 @@ class ClockSampler:
             sm.sort()
             out.update(sm_mhz=sm[len(sm) // 2], sm_max_mhz=max(mx), reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write what the timed path returned in its last step as <out_dir>/<name>.npy — floating-point results as float32,
+    token ids as float64 (exact) — so that two builds can be compared output for output on the same seeded inputs."""
+    import numpy as np
+    host = {name: (t.float() if t.is_floating_point() else t.double()).cpu().numpy() for name, t in arrays.items()}
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def measured_peaks():
@@ -482,7 +499,8 @@ def make_unet_engine(tp_rank=0, tp_size=1, uid=None, seed=0):
 def run_denoise(steps=50, warm_loops=1, timed_loops=1, batch=1, hw=128, seed=0, profile=False, eng=None, sync=None,
                 latent_seed=0):
     """50 Euler steps of the Emu2-Gen denoise loop (CFG, guidance 3, 1024x1024 -> latent 128x128) on random-init weights
-    of the published UNet topology; returns dict(steps_per_s, ms_per_step, launches_per_step, finite, sha1 of the latents).
+    of the published UNet topology, `warm_loops` untimed loops then `timed_loops` timed ones; returns dict(steps_per_s, ms_per_step, launches_per_step, finite, sha1 of the latents,
+    the latents themselves).
     `eng`: a UNet engine (possibly one half of a CFG-parallel pair); `sync`: barrier used around the timed region."""
     import hashlib
     from emu_b200 import _lib
@@ -527,7 +545,7 @@ def run_denoise(steps=50, warm_loops=1, timed_loops=1, batch=1, hw=128, seed=0, 
            "finite": bool(torch.isfinite(lat).all()),
            # correctness handle: the same seeds must give the same latents on 1 GPU and on a CFG-parallel pair (bitwise)
            "latents_sha1": hashlib.sha1(lat.cpu().numpy().tobytes()).hexdigest()[:16],
-           "latents_abs_mean": float(lat.abs().mean())}
+           "latents_abs_mean": float(lat.abs().mean()), "latents": lat}
     if own:
         eng.close()
     return out
@@ -621,6 +639,7 @@ def run_cuda(args):
     launches = _lib.launch_count() - l0
     clocks = sampler.stop() if rank == 0 else {}
     assert toks.shape[1] == NEW_TOKENS, toks.shape
+    outputs = {"tokens": toks}
     value = args.steps * NEW_TOKENS / (ms / 1000.0)
 
     # end to end through the public API with host buffers
@@ -712,7 +731,7 @@ def run_cuda(args):
             except Exception:
                 pass
             if world == 1:
-                r = run_denoise()
+                r = run_denoise(warm_loops=args.warmup, timed_loops=args.steps)
                 images, layout = 1, "1 GPU: UNet batch 2 (cond + uncond)"
             else:
                 import ctypes
@@ -726,7 +745,7 @@ def run_cuda(args):
                 dist.all_gather(alls, mine)
                 puid = bytes(alls[pair * 2].cpu().numpy().tobytes())   # the id made by the even rank of my pair
                 ueng, _ = make_unet_engine(tp_rank=prank, tp_size=2, uid=puid)
-                r = run_denoise(eng=ueng, sync=barrier, latent_seed=pair)
+                r = run_denoise(eng=ueng, sync=barrier, latent_seed=pair, warm_loops=args.warmup, timed_loops=args.steps)
                 t = torch.tensor([r["ms_per_step"]], device="cuda")
                 dist.all_reduce(t, op=dist.ReduceOp.MAX)
                 r["ms_per_step"] = float(t.item())
@@ -738,12 +757,14 @@ def run_cuda(args):
                 r["latents_sha1_per_pair"] = ["%016x" % (int(hs[2 * q].item()) << 1) for q in range(world // 2)]
                 images, layout = world // 2, "%d CFG-parallel pair(s): cond on even ranks, uncond on odd ranks, one image per pair" % (world // 2)
                 ueng.close()
+            outputs["denoise_latents"] = r["latents"]
             sps = images * 1000.0 / r["ms_per_step"]
             ach = images * 2 * UNET_FLOP_PER_SAMPLE_STEP / (r["ms_per_step"] / 1000.0) / 1e12
             denoise = {"metric": "emu2gen_denoise_steps_per_s", "value": sps, "unit": "steps/s", "ms_per_step": r["ms_per_step"],
                        "images_in_flight": images, "scaling": "strong 1->2 (one image), weak beyond (one image per pair)",
                        "config": "SDXL-topology UNet 2.53B, 1024x1024 (latent 128x128), batch 1 + CFG per image, 50 Euler "
                                  "steps, guidance 3, ctx [2,64,1792], bf16, CUDA-graphed fused step; " + layout,
+                       "timed_loops": args.steps, "warmup_loops": args.warmup,   # loops of 50 steps, from --steps / --warmup
                        "gpu_launches_per_step": r["launches_per_step"], "finite": r["finite"],
                        "latents_sha1": r["latents_sha1"], "latents_abs_mean": r["latents_abs_mean"],
                        "pair_latents_identical": r.get("pair_latents_identical"),
@@ -792,6 +813,8 @@ def run_cuda(args):
         "denoise": denoise,
         "beam5": beam5,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     emit(line)
     if world > 1:
         dist.destroy_process_group()
@@ -911,6 +934,8 @@ def run_c4(args):
     except Exception:
         pass
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"tokens": toks})
         emit({
             "metric": "emu2_c4_interleaved_tok_per_s", "value": args.steps * batch * new_tokens / (ms / 1000.0), "unit": "tok/s",
             "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True,
@@ -960,7 +985,8 @@ def run_c5(args):
             dist.barrier()
         torch.cuda.synchronize()
     eng, _ = make_unet_engine()
-    r = run_denoise(eng=eng, sync=barrier, batch=max(mine, 1), latent_seed=rank, warm_loops=1, timed_loops=max(1, args.steps // 2))
+    r = run_denoise(eng=eng, sync=barrier, batch=max(mine, 1), latent_seed=rank, warm_loops=args.warmup,
+                    timed_loops=args.steps)
     eng.close()
     ms_loop = r["ms_per_step"]
     if world > 1:
@@ -973,6 +999,8 @@ def run_c5(args):
     except Exception:
         pass
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"denoise_latents": r["latents"]})
         ach = prompts * 2 * UNET_FLOP_PER_SAMPLE_STEP / (ms_loop / 1000.0) / 1e12
         emit({"metric": "emu2gen_c5_image_steps_per_s", "value": prompts * 1000.0 / ms_loop, "unit": "image-steps/s",
               "n_gpus": world, "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms_loop, "higher_is_better": True,
@@ -1013,8 +1041,9 @@ def main():
     quiet_stdout()
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=3)
-    ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--steps", type=int, default=3,
+                    help="timed steps: generate calls (c2, c4) and 50-step denoise loops (the denoise half of c2, c5)")
+    ap.add_argument("--warmup", type=int, default=3, help="untimed steps of the same kinds before the timed ones")
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--small", action="store_true", help="tiny plumbing config (debug only; never a bench number)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
@@ -1024,7 +1053,14 @@ def main():
                     help="c2 = BASELINE configs[1] (the headline, default); c4 = configs[3]: 8-shot interleaved prompts "
                          "(seq ~4k), batch 4, 5 beams, LLaMA-33B tensor parallel over --gpus (needs >= 2 GPUs for the KV cache); "
                          "c5 = configs[4]: 32 prompts x 50 denoise steps at 1024x1024, the prompt batch sharded over --gpus")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed (greedy token ids; the final latents of "
+                         "the denoise loop) as DIR/<name>.npy, float32 / float64, to compare two builds on the same inputs")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm: the reference arm only times a sample of the work")
     if args.impl == "reference":
         run_reference(args)
         return

@@ -45,7 +45,7 @@ def main():
         emb[inp.input_ids == 32003] = pe
         pos = (inp.attention_mask.cumsum(-1) - 1).masked_fill(inp.attention_mask == 0, 1)
         lo = model.decoder.lm(inputs_embeds=emb, attention_mask=inp.attention_mask, position_ids=pos)
-        out["prefill_logits_last"] = lo.logits[:, -1, :].float()
+        out["prefill_logits_last"] = lo.logits[:, -1, :].float().clone()   # own storage: a view saves all [B, T, vocab] logits
         # generate: new-token ids straight from lm.generate (what EmuModel.generate decodes, emu.py:213-233)
         from emu.emu import GENERATION_CONFIG
         for name, kw in (("greedy", dict(num_beams=1)), ("beam5", dict(num_beams=5, length_penalty=-1)),

@@ -1,4 +1,5 @@
 """Shared test helpers: deterministic reference-format state dicts, tiny configs, a stub tokenizer."""
+import hashlib
 import math
 
 import torch
@@ -74,6 +75,45 @@ def assert_bf16_parity(name, out, ref32, ref16, ratio=PARITY_RATIO, floor=PARITY
     print("\n[parity] %-34s engine-vs-fp32 %.3e | bf16-oracle-vs-fp32 %.3e | ratio %.2f" % (name, e_eng, e_bf, e_eng / max(e_bf, 1e-12)))
     assert e_eng <= max(ratio * e_bf, floor), (name, e_eng, e_bf)
     return e_eng, e_bf
+
+
+def tensor_digest(t, n_sample=512):
+    """Stand-in for a tensor too large to store as a golden fixture: shape, dtype, the SHA-256 of its bytes and a seeded
+    sample of its values (the sample makes a mismatch readable; the hash keeps the comparison bit-exact)."""
+    t = t.detach().contiguous().cpu()
+    flat = t.reshape(-1)
+    idx = torch.randperm(flat.numel(), generator=torch.Generator().manual_seed(0))[:n_sample].clone()
+    return {"shape": tuple(t.shape), "dtype": str(t.dtype), "sha256": hashlib.sha256(t.numpy().tobytes()).hexdigest(),
+            "idx": idx, "sample": flat[idx].clone()}
+
+
+def assert_equal_digest(t, d):
+    """`t` is bitwise equal to the tensor `d` = tensor_digest(...) was made from."""
+    t = t.detach().contiguous().cpu()
+    assert tuple(t.shape) == d["shape"] and str(t.dtype) == d["dtype"], (tuple(t.shape), t.dtype, d["shape"], d["dtype"])
+    s = t.reshape(-1)[d["idx"]]
+    assert torch.equal(s, d["sample"]), "max |diff| on the sampled values: %g" % (s - d["sample"]).abs().max()
+    assert hashlib.sha256(t.numpy().tobytes()).hexdigest() == d["sha256"]
+
+
+def chat_prompt_cases():
+    """Inputs of the chat prompt-assembly comparison (tests/test_host_cpu.py, tests/golden/gen_golden_reference_checks.py):
+    plain messages for _prepare_inputs and (conversation, is_grounding) pairs for _prepare_chat_inputs."""
+    from PIL import Image
+    from emu_b200.emu2.constants import DEFAULT_VIDEO_TOKEN, FAKE_VIDEO_END_TOKEN
+    imgs = [Image.new("RGB", (64 + 10 * i, 48 + 7 * i), (10 * i, 200 - 20 * i, 30 + i)) for i in range(4)]
+    plain = [
+        [imgs[0], "describe"],
+        ["before", imgs[1], "between", imgs[2], "after"],
+        ["watch:", DEFAULT_VIDEO_TOKEN, imgs[0], imgs[1], FAKE_VIDEO_END_TOKEN, "what happens?", imgs[3]],
+        ["text only"],
+    ]
+    chats = [
+        ([[imgs[0], "what is this?"], ["a cat"], ["and this?", imgs[1]]], True),
+        ([["hello"]], False),
+        ([[imgs[2], imgs[3], "compare"], ["they differ"], ["how?"]], False),
+    ]
+    return plain, chats
 
 
 class StubTokenizer:

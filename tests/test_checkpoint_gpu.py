@@ -2,10 +2,7 @@
 the engine by emu_b200/checkpoint.py, must give the engine the same weights as handing it the state dict directly: the
 image tokens and the first-step logits are compared BITWISE.  Formats: a single safetensors file, a torch .bin, an HF sharded
 index (Emu2/emu/conf/llama_config/pytorch_model.bin.index.json style), the Emu1 `{"module": ...}` wrapper, and LoRA adapters in
-the peft key layout merged while streaming (Emu1/inference.py:40-57).
-
-Written after the round's GPU budget was spent: these tests have NOT run on a B200 yet, so they are marked xfail(strict=False)
-— a pass shows up as XPASS, a failure cannot turn the suite red."""
+the peft key layout merged while streaming (Emu1/inference.py:40-57)."""
 import json
 import os
 
@@ -14,8 +11,7 @@ import torch
 
 from helpers import TINY_LLAMA, TINY_VISION, StubTokenizer, make_emu2_state_dict
 
-pytestmark = [pytest.mark.gpu, pytest.mark.xfail(reason="added after the round's GPU budget was spent: not yet run on a B200",
-                                                 strict=False)]
+pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "emu2_tiny.pt")
 
 

@@ -3,10 +3,13 @@ pipeline, the Euler scheduler tables against the oracle restatement, config tran
 import json
 import os
 
-import pytest
 import torch
 
 from oracle import diffusion_oracle as D
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+# the reference's published Emu2-Gen configuration files (tests/golden/gen_golden_reference_checks.py copies them)
+REF_DIFFUSION_CONFIG = os.path.join(GOLDEN, "emu2_diffusion_config")
 
 
 def test_euler_tables_match_oracle():
@@ -77,12 +80,7 @@ def test_image_transform_matches_reference_formula():
 
 def test_unet_config_translation_and_param_count():
     from emu_b200.emu2.diffusion import unet_config_from_json
-    p = "/root/reference/Emu2/emu/conf/diffusion_config/unet/config.json"
-    if os.path.exists(p):
-        cfg = json.load(open(p))
-    else:
-        import bench
-        cfg = bench.emu2_unet_json()
+    cfg = json.load(open(os.path.join(REF_DIFFUSION_CONFIG, "unet", "config.json")))
     u = unet_config_from_json(cfg)
     assert list(u.block_out_channels)[:3] == [320, 640, 1280] and list(u.transformer_layers)[:3] == [0, 2, 10]
     assert u.head_dim == 64 and u.cross_attention_dim == 1792 and u.projection_class_embeddings_input_dim == 3328
@@ -92,43 +90,30 @@ def test_unet_config_translation_and_param_count():
     assert sum(torch.Size(s).numel() for _, s in bench.unet_param_shapes(bench.emu2_unet_json())) == n
 
 
-@pytest.mark.skipif(not __import__("oracle.ref_shim", fromlist=["x"]).available(),
-                    reason="/root/reference only exists in the authoring container")
 def test_chat_prompt_assembly_vs_live_reference():
-    """Prompt strings and image tensors of EmuChatGeneration._prepare_inputs / _prepare_chat_inputs are identical to the
-    UNMODIFIED reference's (Emu2/emu/chat.py:121-195), for plain, interleaved, video and multi-turn (grounding) inputs."""
-    from PIL import Image
-    from oracle import ref_shim
+    """Prompt strings and image tensors of EmuChatGeneration._prepare_inputs / _prepare_chat_inputs are identical to what
+    the UNMODIFIED reference (Emu2/emu/chat.py:121-195) returned (tests/golden/gen_golden_reference_checks.py), for
+    plain, interleaved, video and multi-turn (grounding) inputs; image tensors bitwise, through their SHA-256."""
+    from helpers import assert_equal_digest, chat_prompt_cases
     from emu_b200.emu2.chat import EmuChatGeneration
-    ref_shim.import_emu2()
-    import emu.chat as rchat
-    from emu.constants import DEFAULT_VIDEO_TOKEN, FAKE_VIDEO_END_TOKEN
+    gold = torch.load(os.path.join(GOLDEN, "reference_checks.pt"))["chat"]
     mine = EmuChatGeneration(_FakeModel())
-    ref = rchat.EmuChatGeneration.__new__(rchat.EmuChatGeneration)   # no model needed for prompt assembly
-    ref.transform = rchat.TF.Compose([
-        rchat.TF.Resize((448, 448), interpolation=rchat.TF.InterpolationMode.BICUBIC), rchat.TF.ToTensor(),
-        rchat.TF.Normalize(mean=rchat.OPENAI_DATASET_MEAN, std=rchat.OPENAI_DATASET_STD)])
-    imgs = [Image.new("RGB", (64 + 10 * i, 48 + 7 * i), (10 * i, 200 - 20 * i, 30 + i)) for i in range(4)]
-    plain = [
-        [imgs[0], "describe"],
-        ["before", imgs[1], "between", imgs[2], "after"],
-        ["watch:", DEFAULT_VIDEO_TOKEN, imgs[0], imgs[1], FAKE_VIDEO_END_TOKEN, "what happens?", imgs[3]],
-        ["text only"],
-    ]
-    for inp in plain:
-        a, b = mine._prepare_inputs(inp), ref._prepare_inputs(inp)
-        assert a[0] == b[0] and a[3:] == b[3:]
-        for x, y in ((a[1], b[1]), (a[2], b[2])):
-            assert (x is None) == (y is None) and (x is None or torch.equal(x, y))
-    chats = [
-        ([[imgs[0], "what is this?"], ["a cat"], ["and this?", imgs[1]]], True),
-        ([["hello"]], False),
-        ([[imgs[2], imgs[3], "compare"], ["they differ"], ["how?"]], False),
-    ]
-    for inp, grounding in chats:
-        a, b = mine._prepare_chat_inputs(inp, is_grounding=grounding), ref._prepare_chat_inputs(inp, is_grounding=grounding)
-        assert a[0] == b[0]
-        assert (a[1] is None) == (b[1] is None) and (a[1] is None or torch.equal(a[1], b[1]))
+    plain, chats = chat_prompt_cases()
+
+    def same(x, d):
+        assert (x is None) == (d is None)
+        if x is not None:
+            assert_equal_digest(x, d)
+    assert len(plain) == len(gold["plain"]) and len(chats) == len(gold["chat"])
+    for inp, b in zip(plain, gold["plain"]):
+        a = mine._prepare_inputs(inp)
+        assert a[0] == b["text"] and a[3:] == b["rest"]
+        same(a[1], b["image"])
+        same(a[2], b["video"])
+    for (inp, grounding), b in zip(chats, gold["chat"]):
+        a = mine._prepare_chat_inputs(inp, is_grounding=grounding)
+        assert a[0] == b["text"]
+        same(a[1], b["image"])
 
 
 class _FakeEncoder:
@@ -235,13 +220,11 @@ def test_builtin_diffusion_config_is_the_published_one(tmp_path):
     unet, vae, sched = conf.load_diffusion_config(None)
     assert unet == conf.EMU2_GEN_UNET and vae == conf.EMU2_GEN_VAE and sched == conf.EMU2_GEN_SCHEDULER
     assert bench.emu2_unet_json() == conf.EMU2_GEN_UNET
-    ref_dir = "/root/reference/Emu2/emu/conf/diffusion_config"
-    if os.path.isdir(ref_dir):
-        r_unet, r_vae, r_sched = conf.load_diffusion_config(ref_dir)
-        for mine, ref in ((unet, r_unet), (vae, r_vae), (sched, r_sched)):
-            assert all(ref[k] == v for k, v in mine.items())
-        assert raw(unet_config_from_json(unet)) == raw(unet_config_from_json(r_unet))
-        assert raw(vae_config_from_json(vae)) == raw(vae_config_from_json(r_vae))
+    r_unet, r_vae, r_sched = conf.load_diffusion_config(REF_DIFFUSION_CONFIG)
+    for mine, ref in ((unet, r_unet), (vae, r_vae), (sched, r_sched)):
+        assert all(ref[k] == v for k, v in mine.items())
+    assert raw(unet_config_from_json(unet)) == raw(unet_config_from_json(r_unet))
+    assert raw(vae_config_from_json(vae)) == raw(vae_config_from_json(r_vae))
     (tmp_path / "scheduler").mkdir()
     json.dump(dict(conf.EMU2_GEN_SCHEDULER, steps_offset=0), open(tmp_path / "scheduler" / "scheduler_config.json", "w"))
     u2, v2, s2 = conf.load_diffusion_config(str(tmp_path))

@@ -1,6 +1,6 @@
 """CPU: the oracle restatement (oracle/emu_oracle.py) against the golden outputs of the UNMODIFIED reference
-(tests/golden/emu2_tiny.pt, made by tests/golden/gen_golden.py) and — when /root/reference is present — against the
-reference imported live."""
+(tests/golden/emu2_tiny.pt, made by tests/golden/gen_golden.py; tests/golden/reference_checks.pt, made by
+tests/golden/gen_golden_reference_checks.py)."""
 import os
 
 import numpy as np
@@ -8,8 +8,8 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import TINY_LLAMA, TINY_VISION, make_emu2_state_dict
-from oracle import emu_oracle as O, ref_shim
+from helpers import TINY_LLAMA, make_emu2_state_dict
+from oracle import emu_oracle as O
 
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "emu2_tiny.pt")
 L, NH = TINY_LLAMA["num_hidden_layers"], TINY_LLAMA["num_attention_heads"]
@@ -64,24 +64,20 @@ def test_generate_image_literal_and_cached(gold, sd):
     assert O.rel_err(out2, gold["genimg_mm"]) < 1e-4
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="reference tree not present (GPU box)")
-def test_oracle_vs_live_reference(sd):
-    d = ref_shim.make_llama_config_dir(TINY_LLAMA["hidden_size"], L, NH, TINY_LLAMA["intermediate_size"])
-    vk = dict(TINY_VISION)
-    model = ref_shim.build_emu2_model(vk, d)
-    model.load_state_dict(sd, strict=True)
-    img = torch.randn(1, 3, 56, 56, generator=torch.Generator().manual_seed(5))
-    with torch.no_grad():
-        ref = model.encode_image(img)
-        gi = model.generate_image(text=["two dogs"])
-    assert O.rel_err(O.encode_image(sd, img, patch=14, num_heads=4, layers=2, n_query=4), ref) < 1e-5
-    tok = model.decoder.tokenizer
+@pytest.fixture(scope="module")
+def ref_checks():
+    return torch.load(os.path.join(os.path.dirname(GOLD), "reference_checks.pt"))
 
-    def ids_fn(k):
-        i = tok(["two dogs[IMG]" + "<image>" * k], padding="longest", return_tensors="pt")
-        return i.input_ids, i.attention_mask
-    lit = O.generate_image_regress(sd, ids_fn, 4, layers=L, heads=NH, image_token_id=32003, boi_token_id=32001)
-    assert O.rel_err(lit, gi) < 1e-5
+
+def test_oracle_vs_live_reference(sd, ref_checks):
+    """encode_image and the literal generate_image against the outputs of the UNMODIFIED reference EmuModel on the same
+    weights, fed the ids its own tokenizer produced (tests/golden/gen_golden_reference_checks.py)"""
+    ref = ref_checks["emu2_tiny"]
+    img = torch.randn(1, 3, 56, 56, generator=torch.Generator().manual_seed(5))
+    assert O.rel_err(O.encode_image(sd, img, patch=14, num_heads=4, layers=2, n_query=4), ref["encode_image"]) < 1e-5
+    lit = O.generate_image_regress(sd, lambda k: ref["generate_image_ids"][k], 4, layers=L, heads=NH, image_token_id=32003,
+                                   boi_token_id=32001)
+    assert O.rel_err(lit, ref["generate_image"]) < 1e-5
 
 
 @pytest.mark.parametrize("H,W,S", [(37, 53, 16), (500, 333, 448), (448, 448, 448), (1024, 768, 448), (100, 100, 224),
@@ -102,14 +98,19 @@ def test_preprocess_oracle_vs_torchvision(H, W, S):
     assert np.array_equal(t(pil).numpy(), P.image_transform(img, S, mean, std))
 
 
-def _cformer_golden():
-    g = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "emu1_cformer_tiny.pt"))
+def _cformer_state_dict(g):
+    """the seeded Causal-Former weights a golden file was made with"""
     from oracle import diffusion_oracle as D, t5_oracle as T
     sd = D.random_state_dict(T.param_shapes(g["cfg"], g["enc_w"], g["out_dim"], n_causal=g["n_causal"]), seed=g["seed"])
     for k in sd:
         if k.endswith("Attention.q.weight"):
             sd[k] = sd[k] * 0.125
-    return g, sd
+    return sd
+
+
+def _cformer_golden():
+    g = torch.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "emu1_cformer_tiny.pt"))
+    return g, _cformer_state_dict(g)
 
 
 def test_t5_oracle_vs_reference_golden():
@@ -124,20 +125,23 @@ def test_t5_oracle_vs_reference_golden():
     assert torch.equal(out16, g["out_bf16"])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference only exists in the authoring container")
-def test_t5_oracle_vs_live_reference_t5_base():
-    """Same, against the live reference at the real t5-base dimensions (12 layers, d_model 768) with its own default
-    initialisation — bit-exact."""
+def test_t5_oracle_vs_live_reference_t5_base(ref_checks):
+    """Same, at the real t5-base dimensions (12 layers, d_model 768, 32 causal queries over 257 EVA-CLIP tokens of width
+    1408): the outputs the reference module produced on seeded weights (tests/golden/gen_golden_reference_checks.py) —
+    bit-exact, fp32 and bf16."""
     from oracle import t5_oracle as T
-    CF = ref_shim.import_emu1_causal_former()
-    torch.manual_seed(0)
-    m = CF(None, n_causal=32, vision_width=1408, output_dim=512).eval()
-    x = torch.randn(1, 257, 1408)
-    for dt in (torch.float32, torch.bfloat16):  # the module is created half bf16 / half fp32: make it uniform first
-        m = m.to(dt)
-        sd = {"cformer." + k: v.detach().clone() for k, v in m.state_dict().items()}
-        with torch.no_grad():
-            assert torch.equal(m(x.to(dt)), T.causal_former(sd, x.to(dt)))
+    g = ref_checks["t5_base"]
+    assert g["cfg"] == T.T5_BASE
+    sd = _cformer_state_dict(g)
+    x = torch.randn(*g["img_embeds_shape"], generator=torch.Generator().manual_seed(g["seed"] + 1))
+    threads = torch.get_num_threads()
+    torch.set_num_threads(1)   # at these widths the CPU GEMMs split their sums by thread count: one thread, as the golden run
+    try:
+        for name, dt in (("fp32", torch.float32), ("bf16", torch.bfloat16)):
+            sdt = {k: v.to(dt) for k, v in sd.items()}
+            assert torch.equal(T.causal_former(sdt, x.to(dt)), g["out_" + name]), name
+    finally:
+        torch.set_num_threads(threads)
 
 
 def test_emu1_oracle_vs_reference_golden():
@@ -156,15 +160,14 @@ def test_emu1_oracle_vs_reference_golden():
         assert torch.equal(T.causal_former(sd, feats, emu1_t5_cfg()), g["cformer_out"])
 
 
-@pytest.mark.skipif(not ref_shim.available(), reason="/root/reference only exists in the authoring container")
-def test_emu1_vit_oracle_vs_live_reference():
-    from helpers import EMU1_VIS88
-    vit = ref_shim.build_emu1_vit(EMU1_VIS88)
-    sd = {"visual." + k: v.detach().clone() for k, v in vit.state_dict().items()}
+def test_emu1_vit_oracle_vs_live_reference(ref_checks):
+    """the pre-norm EVA ViT at head width 88 == forward_features of the reference's EVAVisionTransformer on the same seeded
+    weights (tests/golden/gen_golden_reference_checks.py), bit for bit"""
+    from helpers import EMU1_VIS88, emu1_state_dict
+    sd = emu1_state_dict(EMU1_VIS88)
     img = torch.randn(2, 3, 56, 56, generator=torch.Generator().manual_seed(9))
-    with torch.no_grad():
-        ref = vit.forward_features(img)
-    assert torch.equal(ref, O.vit_forward_features(sd, img, patch=14, num_heads=2, layers=2, postnorm=False))
+    assert torch.equal(ref_checks["emu1_vit88"]["forward_features"],
+                       O.vit_forward_features(sd, img, patch=14, num_heads=2, layers=2, postnorm=False))
 
 
 def _emu1_generate_image_oracle(sd, ids, image, vis):
